@@ -15,6 +15,7 @@ BASELINE.json names two things, measured by two legs:
 
   python bench.py [--gpus N --steps K --warmup W]            our arm (CUDA, through the C ABI)
   python bench.py --impl reference [...]                     the reference's CPU path (oracle port) on host cores
+  python bench.py --dump-outputs DIR [...]                   also write the last timed step's outputs to DIR/*.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for every field.
 """
@@ -62,7 +63,12 @@ def parse_args():
     ap.add_argument("--no-staleness", action="store_true", help="skip the 2 / 4 batches-in-flight measurement")
     ap.add_argument("--no-kernel-table", action="store_true", help="N > 1: skip the per-kernel-family timing pass")
     ap.add_argument("--no-graph", action="store_true", help="launch kernel by kernel instead of replaying CUDA graphs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the metric leg's last timed step computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "b200" or args.gpus != 1 or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200, --gpus 1 and --steps >= 1")
+    return args
 
 
 def keyspace_per_gpu(args):
@@ -326,7 +332,30 @@ def kernel_bytes(stats, dim, state):
     }
 
 
-def run_leg(args, torch, dim, B, rows, name, want_kernels, want_parity):
+DUMP_BYTES = 48 << 20  # what --dump-outputs writes at most: 1260 of the 8192 samples at the default shape
+
+
+def dump_outputs(out_dir, torch, SH, sh, out, ids, slot_off, pf, B):
+    """Writes what one training step gave its caller, for a fixed, seeded sample of the batch's samples (the same
+    sample in every slot): `embeddings` [S, n, dim], the pooled f16 embeddings forward returned, as f32; `updated_rows`
+    [S, n, dim + optimizer state], the table entries of those samples' signs after backward applied the step's
+    gradients; `sample_index` [n], the samples drawn.  Two builds given the same arguments can be compared file for
+    file: the inputs are generated from fixed seeds."""
+    S = len(pf)
+    n = max(1, min(B, DUMP_BYTES // (4 * S * (out.shape[2] + sh.entry_len))))
+    idx = np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+    d_idx = torch.from_numpy(idx).to(out.device)
+    signs = SH.add_prefix(ids, slot_off, pf).view(S, B).index_select(1, d_idx).reshape(-1)
+    rows, found = sh.get_entries(signs)
+    assert bool(found.all()), "a sign the step just updated is not in the table"
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"embeddings": out.index_select(1, d_idx).float(), "updated_rows": rows.view(S, idx.size, -1),
+              "sample_index": torch.from_numpy(idx.astype(np.float64))}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
+def run_leg(args, torch, dim, B, rows, name, want_kernels, want_parity, dump_dir=None):
     """One single-GPU leg: table of `rows` resident rows of `dim`, batches of B samples."""
     import ctypes as C
 
@@ -410,6 +439,9 @@ def run_leg(args, torch, dim, B, rows, name, want_kernels, want_parity):
         t1 = time.time()
         ms = e0.elapsed_time(e1)
         clocks = sampler.stop(t0, t1)
+        if dump_dir is not None:  # before the passes below overwrite the output buffers and update the table again
+            k = (K - 1) % n_sets
+            dump_outputs(dump_dir, torch, SH, sh, outs[k], ids_dev[k], slot_off, pf, B)
         reps = []
         for _ in range(3):  # run-to-run spread of the same K steps
             e0.record(stream)
@@ -716,7 +748,7 @@ def single_gpu(args, torch):
     roof_leg = None
     if not args.no_roofline_leg:
         roof_leg = run_leg(args, torch, 64, 4096, rows, "roofline leg (configs[1])", True, not args.no_parity)
-    leg = run_leg(args, torch, args.dim, args.batch, rows, "metric leg", True, not args.no_parity)
+    leg = run_leg(args, torch, args.dim, args.batch, rows, "metric leg", True, not args.no_parity, args.dump_outputs)
     B, K = args.batch, args.steps
     S = args.slots
     n_occ = S * B

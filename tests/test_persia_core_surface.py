@@ -1,14 +1,12 @@
-"""CPU: the `persia_core` surface (SURVEY.md §8b).  Checks the module layout `persia/prelude.py` expects and
-— when the reference checkout is present (this container, not the GPU box) — runs the reference's OWN Python
-package unchanged on top of it, repeating the assertions of the reference's test/embedding/test_data.py."""
+"""CPU: the `persia_core` surface (SURVEY.md §8b).  Checks the module layout `persia/prelude.py` expects and replays
+what the reference's OWN Python package, run unchanged on top of this surface, read from it and called on it (its
+data / optim classes, and its test/embedding/test_data.py), recorded in tests/golden/persia_core_calls.json."""
 import os
 import sys
 import types
 
 import numpy as np
 import pytest
-
-REF = "/root/reference"
 
 
 @pytest.fixture()
@@ -82,40 +80,76 @@ def test_prefix_rule_and_batch_semantics(pc):
         fwd.get_batch(5)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "persia")), reason="reference checkout not present")
-def test_reference_python_package_runs_on_the_surface(pc, monkeypatch):
-    """`import persia` (the reference's package, unmodified, read from /root/reference) with our persia_core."""
-    if "colorlog" not in sys.modules:
-        try:
-            import colorlog  # noqa: F401
-        except ImportError:  # the reference's logger wants colorlog; give it a plain formatter
-            import logging
+def _decode(v, objs):
+    if isinstance(v, dict):
+        (kind, x), = v.items()
+        if kind == "handle":
+            return objs[x]
+        if kind == "bytes":
+            return bytes.fromhex(x)
+        if kind == "ndarray":
+            return np.array(x["data"], dtype=np.dtype(x["dtype"])).reshape(x["shape"])
+        if kind == "dtype":
+            return np.dtype(x)
+        if kind == "nptype":
+            return np.dtype(x).type
+        if kind == "npscalar":
+            return np.dtype(x["dtype"]).type(x["value"])
+        if kind in ("list", "tuple"):
+            return (list if kind == "list" else tuple)(_decode(e, objs) for e in x)
+        raise ValueError(kind)
+    return v
 
-            m = types.ModuleType("colorlog")
-            m.ColoredFormatter = lambda fmt=None, *a, **k: logging.Formatter("%(levelname)s %(message)s")
-            monkeypatch.setitem(sys.modules, "colorlog", m)
-    monkeypatch.syspath_prepend(REF)
-    for k in [k for k in sys.modules if k == "persia" or k.startswith("persia.")]:
-        monkeypatch.delitem(sys.modules, k)
-    import persia  # noqa: F401
-    from persia.embedding import EmbeddingConfig
-    from persia.embedding.data import IDTypeFeature, IDTypeFeatureWithSingleID, Label, NonIDTypeFeature, PersiaBatch
-    from persia.embedding.optim import SGD, Adagrad, Adam
 
-    # test/embedding/test_data.py of the reference
-    batch_size = 5
-    for dt in (np.bool_, np.int8, np.int16, np.int32, np.int64, np.float32, np.float64, np.uint8):
-        NonIDTypeFeature(np.zeros((batch_size, 3), dtype=dt))
-    ids = [IDTypeFeature("f1", [np.array([1, 2], np.uint64) for _ in range(batch_size)]),
-           IDTypeFeatureWithSingleID("f2", np.arange(batch_size, dtype=np.uint64))]
-    with pytest.raises(Exception):  # requires_grad without labels
-        PersiaBatch(ids, requires_grad=True)
-    pb = PersiaBatch(ids, non_id_type_features=[NonIDTypeFeature(np.ones((batch_size, 2), np.float32))],
-                     labels=[Label(np.ones((batch_size, 1), np.float32))], requires_grad=True, meta=b"m")
-    assert isinstance(pb.to_bytes(), bytes)
-    SGD(0.1).optimizer_base, Adagrad(0.1).optimizer_base, Adam(1e-3).optimizer_base  # noqa: B018
-    cfg = EmbeddingConfig()
-    assert cfg.weight_bound == 10 and cfg.admit_probability == 1.0
+def _replay(scenario):
+    """Replays, against this persia_core, every name the reference's `persia` package read from persia_core and every
+    call it made, in order, checking each call's outcome: the type it returned or the exception it raised
+    (tests/golden/persia_core_calls.json, recorded by tests/golden/make_persia_core_calls.py)."""
+    import json
+
+    fx = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "persia_core_calls.json")))
+    events = fx["scenarios"][scenario]
+    objs = {}
+
+    def resolve(target):
+        head, *rest = target.split(".")
+        obj = objs[int(head[1:])] if head.startswith("$") else sys.modules[head]
+        for part in rest:
+            obj = getattr(obj, part)
+        return obj
+
+    n_calls = 0
+    for k, ev in enumerate(events):
+        where = f"event {k}: {ev['target']}"
+        if ev["op"] == "getattr":
+            v = resolve(ev["target"])
+            assert "type" not in ev or type(v).__name__ == ev["type"], where
+            continue
+        fn = resolve(ev["target"])
+        args = [_decode(a, objs) for a in ev["args"]]
+        kwargs = {key: _decode(a, objs) for key, a in ev["kwargs"].items()}
+        want = ev["result"]
+        n_calls += 1
+        if "raises" in want:
+            with pytest.raises(Exception) as e:
+                fn(*args, **kwargs)
+            assert type(e.value).__name__ == want["raises"], where
+            continue
+        r = fn(*args, **kwargs)
+        if "handle" in want:
+            objs[want["handle"]] = r
+        else:
+            assert type(r).__name__ == want["type"], where
+    return n_calls
+
+
+def test_reference_python_package_runs_on_the_surface(pc):
+    """What the reference's own `persia` package (persia/prelude.py, persia/embedding/{data,optim}.py) asks of
+    persia_core when its data, optimizer and config classes are driven: the batch assembly with ids, dense features,
+    labels and meta, the requires_grad-without-labels refusal, serialisation, and the three optimizer inits."""
+    assert _replay("package_surface") == 18
+
+
 
 
 def test_farmhash_numpy_matches_golden(pc):
@@ -131,28 +165,8 @@ def test_farmhash_numpy_matches_golden(pc):
     assert [g.tolist() for g in got] == [list(v) for v in fx["hashstack_rounds2_size10"].values()]
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "test", "embedding", "test_data.py")),
-                    reason="reference checkout not present")
-def test_reference_own_test_file_passes_unmodified(tmp_path):
-    """The reference's test/embedding/test_data.py, run by pytest as it stands in /root/reference, with this repo's
-    persia_core registered in place of the Rust extension (a subprocess: clean module state, cwd outside both trees)."""
-    import subprocess
-
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    prelude = (
-        "import sys, types, logging\n"
-        "try:\n"
-        "    import colorlog\n"
-        "except ImportError:\n"  # the reference's logger wants colorlog; give it a plain formatter
-        "    m = types.ModuleType('colorlog')\n"
-        "    m.ColoredFormatter = lambda fmt=None, *a, **k: logging.Formatter('%(levelname)s %(message)s')\n"
-        "    sys.modules['colorlog'] = m\n"
-        "from persia_b200 import persia_core\n"
-        "persia_core.install()\n"
-        "import pytest\n"
-        f"sys.exit(pytest.main(['-q', '-p', 'no:cacheprovider', {os.path.join(REF, 'test', 'embedding', 'test_data.py')!r}]))\n"
-    )
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([root, REF]), PYTHONDONTWRITEBYTECODE="1")
-    r = subprocess.run([sys.executable, "-c", prelude], cwd=tmp_path, env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "5 passed" in r.stdout
+def test_reference_own_test_file_passes_unmodified(pc):
+    """What the reference's test/embedding/test_data.py (5 tests, all passing on this persia_core when recorded) asks
+    of persia_core: check_pyarray_dtype_valid over every supported dtype, the requires_grad-without-labels refusal and
+    serialisation."""
+    assert _replay("reference_test_data") == 15
