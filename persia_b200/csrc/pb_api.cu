@@ -112,8 +112,10 @@ struct pb_ctx {
   uint32_t* nan_tick = nullptr;
   float* vw_stage = nullptr;
   size_t vw_stage_floats = 0;
-  cudaStream_t side = nullptr;  // hot items + scratch-set clearing run beside the main stream during pb_backward
-  cudaStream_t side2 = nullptr;  // the warm items, beside the cold ones
+  float* hot_stage = nullptr;  // [b.hot_cap][hot_stage_stride(dim)] reduced gradients of the hot items
+  size_t hot_stage_floats = 0;
+  cudaStream_t side = nullptr;  // hot items run beside the main stream during pb_backward
+  cudaStream_t side2 = nullptr;  // scratch-set clearing and the warm items, beside the cold ones
   cudaEvent_t ev_fork = nullptr, ev_nan = nullptr, ev_join = nullptr, ev_join2 = nullptr;
   // raw slot (pb_forward_raw / pb_backward_raw): allocated on first use
   uint32_t* occ_cell = nullptr;
@@ -603,7 +605,7 @@ int pb_ctx_destroy(pb_ctx* c) {
   cudaDeviceSynchronize();
   drop_pending(c);
   void* ptrs[] = {c->b.set,   c->b.occ_set, c->b.item_cell, c->b.seg_occ, c->b.cold, c->b.warm, c->b.hot, c->b.hot_bits, c->b.cnt,
-                  c->occ_cell, c->occ_outrow, c->row_off, c->nan_tick, c->vw_stage, c->dev_tick, c->raw.set,
+                  c->occ_cell, c->occ_outrow, c->row_off, c->nan_tick, c->vw_stage, c->hot_stage, c->dev_tick, c->raw.set,
                   c->raw.occ_set, c->raw.flag, c->raw.rank, c->raw.tiles, c->raw.distinct_cell, c->raw.counts, c->raw_stage};
   for (void* p : ptrs)
     if (p) cudaFree(p);
@@ -763,19 +765,15 @@ int pb_backward(pb_table* t, pb_ctx* c, const void* const* h_grads, int is_f16, 
     }
     vw = c->vw_stage;
   }
-  // beside the main stream: the scratch set is emptied and, once the NaN marks are known, the hot items are reduced
-  PB_CUDA(cudaEventRecord(c->ev_fork, st));
-  PB_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-  if (c->set_dirty) {
-    launch_clear_items(c->b, c->side);
-    c->set_dirty = false;
+  const size_t hot_need = (size_t)c->b.hot_cap * hot_stage_stride(t->d.dim);
+  if (hot_need > c->hot_stage_floats) {
+    PB_CUDA(cudaStreamSynchronize(st));
+    if (c->hot_stage) cudaFree(c->hot_stage);
+    c->hot_stage = nullptr;
+    c->hot_stage_floats = 0;
+    PB_CUDA(cudaMalloc(&c->hot_stage, sizeof(float) * hot_need));
+    c->hot_stage_floats = hot_need;
   }
-  uint32_t elems = c->batch * t->d.dim;
-  launch_nan_scan(gr, S, elems, is_f16 != 0, c->dev_tick, c->nan_tick, d_slot_status, st);
-  if (adam_keys.n) launch_adam_advance(t->adam_dev, adam_keys, t->op.b1, t->op.b2, st, &gr, S, c->dev_tick, c->nan_tick);
-  PB_CUDA(cudaEventRecord(c->ev_nan, st));
-  PB_CUDA(cudaStreamWaitEvent(c->side, c->ev_nan, 0));
-  PB_CUDA(cudaStreamWaitEvent(c->side2, c->ev_nan, 0));
   ReduceArgs a;
   std::memset(&a, 0, sizeof(a));
   a.b = c->b;
@@ -785,17 +783,42 @@ int pb_backward(pb_table* t, pb_ctx* c, const void* const* h_grads, int is_f16, 
   a.tick_ptr = c->dev_tick;
   a.nan_tick = c->nan_tick;
   a.vw_stage = vw;
+  a.hot_stage = c->hot_stage;
+  a.hot_stride = hot_stage_stride(t->d.dim);
   a.batch = c->batch;
   a.quiet_miss = 0;
-  for (uint32_t r = 0; r < c->n_rounds; ++r) {
+  auto set_round = [&](uint32_t r) {
     a.round = r;
     std::memset(a.round_mask, 0, sizeof(a.round_mask));
     for (uint32_t s = 0; s < S; ++s)
       if (c->round_of[s] == r) a.round_mask[s >> 5] |= 1u << (s & 31);
-    // one round (no shared feature groups, the usual case): hot items run beside the others; several: one after another
-    // the items of a round are distinct rows, whatever their list.
-    const bool one = c->n_rounds == 1 && !profiling();  // (timed alone when the bench instruments a family)
-    launch_reduce_items(t->d, t->op, t->hy, sl, gr, is_f16 != 0, a, st, one ? c->side : st, one ? c->side2 : st, false);
+  };
+  // One round (no shared feature groups, the usual case): the hot items' sums (the long pole) start on `side` at once,
+  // beside the NaN scan, and their steps follow the verdict; warm items run on side2 beside the cold ones.  Several
+  // rounds: one kernel after another, round by round (the items of a round are distinct rows, whatever their list).
+  const bool one = c->n_rounds == 1 && !profiling();  // (timed alone when the bench instruments a family)
+  PB_CUDA(cudaEventRecord(c->ev_fork, st));
+  PB_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
+  PB_CUDA(cudaStreamWaitEvent(c->side2, c->ev_fork, 0));
+  if (c->set_dirty) {  // nothing in the backward reads the scratch set
+    launch_clear_items(c->b, c->side2);
+    c->set_dirty = false;
+  }
+  if (one) {
+    set_round(0);
+    launch_reduce_hot(t->d, sl, gr, is_f16 != 0, a, c->side);
+  }
+  uint32_t elems = c->batch * t->d.dim;
+  launch_nan_scan(gr, S, elems, is_f16 != 0, c->dev_tick, c->nan_tick, d_slot_status, st);
+  if (adam_keys.n) launch_adam_advance(t->adam_dev, adam_keys, t->op.b1, t->op.b2, st, &gr, S, c->dev_tick, c->nan_tick);
+  PB_CUDA(cudaEventRecord(c->ev_nan, st));
+  PB_CUDA(cudaStreamWaitEvent(c->side, c->ev_nan, 0));
+  PB_CUDA(cudaStreamWaitEvent(c->side2, c->ev_nan, 0));
+  for (uint32_t r = 0; r < c->n_rounds; ++r) {
+    set_round(r);
+    if (!one) launch_reduce_hot(t->d, sl, gr, is_f16 != 0, a, st);
+    launch_step_hot(t->d, t->op, t->hy, sl, gr, a, one ? c->side : st);
+    launch_reduce_items(t->d, t->op, t->hy, sl, gr, is_f16 != 0, a, st, one ? c->side2 : st, false);
   }
   PB_CUDA(cudaEventRecord(c->ev_join, c->side));
   PB_CUDA(cudaStreamWaitEvent(st, c->ev_join, 0));
@@ -1040,8 +1063,9 @@ int pb_backward_sharded(pb_table* t, pb_ctx* c, pb_xchg* x, const void* const* h
   for (uint32_t s = 0; s < S; ++s) a.round_mask[s >> 5] |= 1u << (s & 31);
   a.x = x->d;
   PB_CUDA(cudaStreamWaitEvent(c->side2, c->ev_nan, 0));
-  launch_reduce_items(t->d, t->op, t->hy, sl, gr, is_f16 != 0, a, st, profiling() ? st : c->side, profiling() ? st : c->side2,
-                      true);  // requester: gradients -> owners' areas
+  // requester: gradients -> owners' areas
+  launch_reduce_hot(t->d, sl, gr, is_f16 != 0, a, profiling() ? st : c->side, true);
+  launch_reduce_items(t->d, t->op, t->hy, sl, gr, is_f16 != 0, a, st, profiling() ? st : c->side2, true);
   PB_CUDA(cudaEventRecord(c->ev_join, c->side));
   PB_CUDA(cudaStreamWaitEvent(st, c->ev_join, 0));
   PB_CUDA(cudaEventRecord(c->ev_join2, c->side2));

@@ -109,6 +109,8 @@ struct ReduceArgs {
   const uint32_t* tick_ptr;
   const uint32_t* nan_tick;
   float* vw_stage;             // Adagrad vectorwise: one reduced gradient per item
+  float* hot_stage;            // [hot_cap][hot_stride] reduced gradient of every hot item (k_reduce_hot -> k_step_hot)
+  uint32_t hot_stride;
   uint32_t batch, round, quiet_miss;
   uint32_t round_mask[PB_MAX_SLOTS / 32];  // slots stepped by this launch (slots of one feature group take turns)
   XchgDev x;                   // sharded: the reduced gradient is stored into the owner's receive area instead
@@ -150,10 +152,17 @@ void launch_copy_entries(bool write, const TableDev& t, const uint32_t* occ_cell
                          uint8_t* found, cudaStream_t st);
 void launch_nan_scan(const GradsDev& gr, uint32_t n_slots, uint32_t elems_per_slot, bool f16, const uint32_t* tick,
                      uint32_t* nan_tick, int32_t* status, cudaStream_t st);
-// pb_reduce.cu: cold + warm items on `st`, hot items on `st_hot` (may equal st)
-// send: sharded requester — a.x names the owners' receive areas, no row is touched here
+// pb_reduce.cu.  send: sharded requester — a.x names the owners' receive areas, no row is touched here.
+// Hot items: their gradient sums go to a.hot_stage (to the owners when sending); the sums read no NaN verdict, so they
+// may start before the NaN scan has finished.  launch_step_hot then steps the rows of the applied ones.
+void launch_reduce_hot(const TableDev& t, const SlotsDev& sl, const GradsDev& gr, bool f16, const ReduceArgs& a,
+                       cudaStream_t st, bool send = false);
+void launch_step_hot(const TableDev& t, const OptimDev& op, const HyperDev& hy, const SlotsDev& sl, const GradsDev& gr,
+                     const ReduceArgs& a, cudaStream_t st);
+uint32_t hot_stage_stride(uint32_t dim);
+// cold items on `st`, warm items on `st_warm` (may equal st)
 void launch_reduce_items(const TableDev& t, const OptimDev& op, const HyperDev& hy, const SlotsDev& sl,
-                         const GradsDev& gr, bool f16, const ReduceArgs& a, cudaStream_t st, cudaStream_t st_hot, cudaStream_t st_warm,
+                         const GradsDev& gr, bool f16, const ReduceArgs& a, cudaStream_t st, cudaStream_t st_warm,
                          bool send = false);
 // pb_shard.cu
 void launch_route_items(bool training, const SlotsDev& sl, const BatchDev& b, const XchgDev& x, cudaStream_t st);

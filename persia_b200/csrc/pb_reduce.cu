@@ -14,12 +14,12 @@
 //                   whole chip's worth of groups resident.
 //   k_reduce_warm   a lane group per item: the group sorts the item's <= 32 occurrences in shared memory (rank by
 //                   counting), then adds them in order.
-//   k_reduce_hot    persistent; a two-warp CTA per item.  The occurrences are put in order by setting one bit per
-//                   occurrence in a shared-memory bitmap over the slot's sample range (a counting sort that costs
-//                   B/32 words).  Warp 0 streams the gradient rows, 32 per stage, into a shared-memory ring with
-//                   cp.async.bulk (one bulk copy per row, completion on the stage's mbarrier); warp 1 waits on the
-//                   stage and adds its rows in order — a dependent FADD chain fed from shared memory, which is the
-//                   floor for a strictly sequential sum — then performs the optimizer step.
+//   k_reduce_hot    persistent; a CTA per item.  The occurrences are put in order from a bitmap over the slot's
+//                   samples (a counting sort that costs B/32 words); producer warps stream the gradient rows into a
+//                   shared-memory ring, chain warps add them in order — a dependent FADD chain fed from shared memory,
+//                   which is the floor for a strictly sequential sum — and store the sum to the hot stage.  It reads no
+//                   NaN verdict, so it runs beside the NaN scan.
+//   k_step_hot      a warp per hot item, after the NaN verdict: the optimizer step with the staged sum.
 #include <cstdlib>
 
 #include "pb_optim.cuh"
@@ -159,13 +159,17 @@ __device__ __forceinline__ uint32_t* send_gok_ptr(const XchgDev& x, uint32_t tar
   return reinterpret_cast<uint32_t*>(x.base[q] + x.off_gok) + ((size_t)x.rank * x.cap + k);
 }
 
-// slots whose gradient is skipped or holds a NaN (mod.rs:731-746), or that this launch does not step, as a bit mask
-__device__ __forceinline__ void build_dead_mask(uint32_t* dead, const GradsDev& gr, const ReduceArgs& a, uint32_t n_slots) {
+// slots whose gradient is skipped or holds a NaN (mod.rs:731-746), or that this launch does not step, as a bit mask.
+// with_nan = false: only what the host knows (no gradient, not this round) — the NaN verdict is not read, so the kernel
+// need not wait for the scan.
+__device__ __forceinline__ void build_dead_mask(uint32_t* dead, const GradsDev& gr, const ReduceArgs& a, uint32_t n_slots,
+                                                bool with_nan = true) {
   if (threadIdx.x < PB_MAX_SLOTS / 32) dead[threadIdx.x] = 0u;
   __syncthreads();
-  const uint32_t tick = *a.tick_ptr;
+  const uint32_t tick = with_nan ? *a.tick_ptr : 0u;
   for (uint32_t s = threadIdx.x; s < PB_MAX_SLOTS; s += blockDim.x) {
-    const bool off = s >= n_slots || !gr.ptr[s] || a.nan_tick[s] == tick || !((a.round_mask[s >> 5] >> (s & 31)) & 1u);
+    const bool off = s >= n_slots || !gr.ptr[s] || (with_nan && a.nan_tick[s] == tick) ||
+                     !((a.round_mask[s >> 5] >> (s & 31)) & 1u);
     if (off) atomicOr(&dead[s >> 5], 1u << (s & 31));
   }
   __syncthreads();
@@ -350,7 +354,8 @@ __global__ void __launch_bounds__(256) k_reduce_cold(TableDev t, OptimDev op, Hy
 //              chunk's ring slot; every lane arrives on the slot's `full` mbarrier.  The common case (one id per
 //              sample, no scaling) has its own lean loop: ~25 instructions per 16 bytes is what bounds a producer.
 //   chain      (CH warps, 32 * EPL columns each) waits for the slot and adds its rows in order: one LDS and EPL
-//              dependent FADDs per row — nothing else — then arrives on `empty`; finally the optimizer step.
+//              dependent FADDs per row — nothing else — then arrives on `empty`; finally it stores the sum to the item's
+//              row of the hot stage (k_step_hot steps it once the NaN verdict is known) or, sharded, to the owner.
 // Measured alternatives (profiles/r2_hot_ubench_*.txt): cp.async.bulk of the rows into a raw ring + converter warps is
 // bound by the copy engine's issue rate (~60 cycles per 128-byte copy and SM), a single warp doing load + convert + add
 // by the instruction stream (~40 cycles per row).
@@ -570,9 +575,15 @@ __device__ __forceinline__ void chain_block(float (&acc)[EPL], const float* rp, 
   }
 }
 
+// entry of `hot` of the h-th hot item in reduce order: the giants, the huge ones (both listed from the list's end), the rest
+__device__ __forceinline__ uint32_t hot_entry(const BatchDev& b, uint32_t h, uint32_t n_giant, uint32_t n_huge) {
+  return h < n_giant ? b.hot_cap - 1u - h
+                     : (h < n_giant + n_huge ? b.hot_cap - 1u - b.giant_cap - (h - n_giant) : h - n_giant - n_huge);
+}
+
 template <int EPL, bool F16, bool SEND>
-__global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, OptimDev op, HyperDev hy, SlotsDev sl, GradsDev gr,
-                                                              ReduceArgs a, HotGeom geo, unsigned long long* trace) {
+__global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, SlotsDev sl, GradsDev gr, ReduceArgs a, HotGeom geo,
+                                                              unsigned long long* trace) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint32_t dead[PB_MAX_SLOTS / 32];
   __shared__ uint32_t s_item, s_nwin;
@@ -580,7 +591,6 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
   __shared__ uint16_t sorted[HOT_WIN];
   __shared__ __align__(8) uint64_t bars[2 * HOT_MAX_SLOTS];  // full[0..8), empty[8..16)
   float* ring = reinterpret_cast<float*>(smem_raw);                     // [S][R][stride] prepared rows
-  float* vstage = ring + (size_t)geo.S * geo.R * geo.stride;            // [dim] Adagrad-vectorwise dot
   const uint32_t tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // PW producers share S slots: PW <= S keeps a producer from running two rounds ahead of the chain (the parity of a
   // slot's barrier only tells odd rounds from even ones)
@@ -592,7 +602,8 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  build_dead_mask(dead, gr, a, sl.n_slots);  // ends with __syncthreads
+  // sending: the owner is told whether to apply, which needs the NaN verdict; staging: k_step_hot decides
+  build_dead_mask(dead, gr, a, sl.n_slots, SEND);  // ends with __syncthreads
   const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + HOT_MAX_SLOTS);
   const uint32_t n_giant = a.b.cnt[BC_GIANT], n_huge = a.b.cnt[BC_HUGE];  // the longest chains first
   const uint32_t n_hot = a.b.cnt[BC_HOT] + n_huge + n_giant;
@@ -607,8 +618,8 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
     const uint32_t h = s_item;
     if (h >= n_hot) break;
     if (trace && tid == 0) trace[8 * h] = globaltimer_ns();
-    const uint4 d = a.b.hot[h < n_giant ? a.b.hot_cap - 1u - h
-                                        : (h < n_giant + n_huge ? a.b.hot_cap - 1u - a.b.giant_cap - (h - n_giant) : h - n_giant - n_huge)];
+    const uint32_t entry = hot_entry(a.b, h, n_giant, n_huge);
+    const uint4 d = a.b.hot[entry];
     const uint32_t row = d.x, cnt = d.z, slot = d.w;
     const bool bm_mode = d.y >> 31;
     const uint32_t base = d.y & 0x7FFFFFFFu;  // first bitmap word of the item, or first entry of its occurrence list
@@ -618,8 +629,7 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
       skip = row == ROW_NONE || slot_dead(dead, slot);
       if (row != ROW_NONE && tid == 0) *send_gok_ptr(a.x, row) = slot_dead(dead, slot) ? 0u : 1u;
     } else {
-      skip = slot_dead(dead, slot) || row >= t.capacity;
-      if (!slot_dead(dead, slot) && row >= t.capacity && tid == 0 && !a.quiet_miss) atomicAdd(&t.counters[CTR_GRAD_MISS], 1u);
+      skip = slot_dead(dead, slot) || row >= t.capacity;  // (k_step_hot counts the miss)
     }
     if (skip) {  // the item's bits must still go back to zero for the next batch
       if (bm_mode)
@@ -627,10 +637,7 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
       continue;
     }
     const ItemSrc src = item_src(sl, gr, a, slot);
-    float* prow = SEND ? send_grad_ptr(a.x, row, t.dim) : t.rows + (size_t)row * t.stride;
-    StepCtx sc;
-    sc.vw_state = sc.r1 = sc.r2 = 0.0f;
-    if (!SEND) sc = step_ctx(prow, t, op, gr, slot);
+    float* dst = SEND ? send_grad_ptr(a.x, row, t.dim) : a.hot_stage + (size_t)entry * a.hot_stride;
     for (uint32_t pass = 0; pass < n_pass; ++pass) {
       const uint32_t col0 = pass * HOT_COLS;
       HotGeom g = geo;
@@ -762,43 +769,68 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) k_reduce_hot(TableDev t, Optim
         trace[8 * h + 2] = globaltimer_ns();
         trace[8 * h + 3] = ((unsigned long long)blockIdx.x << 32) | cnt;
       }
-      // ---- the optimizer step on this pass's columns (chain warps).  Columns past dim (dim % EPL != 0) were summed
-      // from the ring's padding and are dropped here.
+      // ---- this pass's columns of the sum (chain warps).  Columns past dim (dim % EPL != 0) were summed from the
+      // ring's padding and are dropped here.
       if (own) {
         const uint32_t nq = min((uint32_t)EPL, t.dim - e0);
-        if (SEND) {
-          if (nq == EPL) RowElems<-1, EPL>::template st<EPL>(prow + e0, acc);
-          else for (uint32_t q = 0; q < nq; ++q) prow[e0 + q] = acc[q];
-        } else if (nq == EPL) {
-          RowElems<-1, EPL> rc;
-          rc.load(prow, e0, t, op);
-          if (op.kind == PB_OPT_ADAGRAD_VW) {
-#pragma unroll
-            for (int q = 0; q < EPL; ++q) vstage[e0 + q] = acc[q];
-          }
-          rc.step(e0, acc, t, op, hy, sc);
-          rc.store(prow, e0, t, op);
-        } else {
-          for (uint32_t q = 0; q < nq; ++q) {
-            RowElems<-1, 1> rc;
-            float one[1] = {acc[q]};
-            rc.load(prow, e0 + q, t, op);
-            if (op.kind == PB_OPT_ADAGRAD_VW) vstage[e0 + q] = acc[q];
-            rc.step(e0 + q, one, t, op, hy, sc);
-            rc.store(prow, e0 + q, t, op);
-          }
-        }
-      }
-    }
-    if (!SEND && op.kind == PB_OPT_ADAGRAD_VW) {  // state = state*mom + dot(g,g)/dim (optim.rs:280-283)
-      __syncthreads();                            // every chain warp staged its columns
-      if (tid == 0) {
-        float gs = __fdiv_rn(vw_dot(vstage, t.dim), (float)t.dim);
-        prow[t.dim] = __fadd_rn(__fmul_rn(sc.vw_state, op.mom), gs);
+        if (nq == EPL) RowElems<-1, EPL>::template st<EPL>(dst + e0, acc);
+        else for (uint32_t q = 0; q < nq; ++q) dst[e0 + q] = acc[q];
       }
     }
   }
   if (failed && lane == 0) atomicAdd(&t.counters[CTR_ERR], 1u);
+}
+
+// ---- the optimizer step of the hot items, once the NaN verdict is known: a warp per item, the reduced gradient from the
+// hot stage.  Lane l owns the elements e0 = (l + 32 k) * EPL, EPL at a time and the last ones one by one.  When dim is
+// not a multiple of EPL the state arrays (row + dim, row + 2 dim) are not EPL-float aligned: every element goes one by
+// one then.  (An element's step depends on its index alone, so the grouping never changes a result.)
+template <int EPL>
+__global__ void __launch_bounds__(256) k_step_hot(TableDev t, OptimDev op, HyperDev hy, SlotsDev sl, GradsDev gr, ReduceArgs a) {
+  __shared__ uint32_t dead[PB_MAX_SLOTS / 32];
+  const uint32_t n_giant = a.b.cnt[BC_GIANT], n_huge = a.b.cnt[BC_HUGE];
+  const uint32_t n_hot = a.b.cnt[BC_HOT] + n_huge + n_giant;
+  const uint32_t per_block = blockDim.x / 32u;
+  if (blockIdx.x * per_block >= n_hot) return;  // whole block
+  build_dead_mask(dead, gr, a, sl.n_slots);
+  const uint32_t lane = threadIdx.x & 31u;
+  for (uint32_t h = blockIdx.x * per_block + threadIdx.x / 32u; h < n_hot; h += gridDim.x * per_block) {
+    const uint32_t entry = hot_entry(a.b, h, n_giant, n_huge);
+    const uint4 d = a.b.hot[entry];
+    const uint32_t row = d.x, slot = d.w;
+    if (slot_dead(dead, slot)) continue;
+    if (row >= t.capacity) {
+      if (lane == 0 && !a.quiet_miss) atomicAdd(&t.counters[CTR_GRAD_MISS], 1u);  // gradient_id_miss_count (PS mod.rs:401-403)
+      continue;
+    }
+    const float* g = a.hot_stage + (size_t)entry * a.hot_stride;
+    float* prow = t.rows + (size_t)row * t.stride;
+    const StepCtx sc = step_ctx(prow, t, op, gr, slot);
+    const bool aligned = t.dim % EPL == 0;
+    for (uint32_t e0 = lane * EPL; e0 < t.dim; e0 += 32u * EPL) {
+      const uint32_t nq = min((uint32_t)EPL, t.dim - e0);
+      if (aligned && nq == EPL) {
+        float acc[EPL];
+        RowElems<-1, EPL>::template ld<EPL>(g + e0, acc);
+        RowElems<-1, EPL> rc;
+        rc.load(prow, e0, t, op);
+        rc.step(e0, acc, t, op, hy, sc);
+        rc.store(prow, e0, t, op);
+      } else {
+        for (uint32_t q = 0; q < nq; ++q) {
+          RowElems<-1, 1> rc;
+          float one[1] = {g[e0 + q]};
+          rc.load(prow, e0 + q, t, op);
+          rc.step(e0 + q, one, t, op, hy, sc);
+          rc.store(prow, e0 + q, t, op);
+        }
+      }
+    }
+    if (op.kind == PB_OPT_ADAGRAD_VW) {  // state = state*mom + dot(g,g)/dim (optim.rs:280-283)
+      __syncwarp();                      // every lane has read the old state (step_ctx)
+      if (lane == 0) prow[t.dim] = __fadd_rn(__fmul_rn(sc.vw_state, op.mom), __fdiv_rn(vw_dot(g, t.dim), (float)t.dim));
+    }
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -830,8 +862,8 @@ static unsigned long long* g_hot_trace = nullptr;  // debugging aid: per hot ite
 void set_hot_trace(unsigned long long* p) { g_hot_trace = p; }
 
 template <int EPL, bool F16, bool SEND>
-static void hot_launch(const TableDev& t, const OptimDev& op, const HyperDev& hy, const SlotsDev& sl, const GradsDev& gr,
-                       const ReduceArgs& a, uint32_t vec, cudaStream_t st) {
+static void hot_launch(const TableDev& t, const SlotsDev& sl, const GradsDev& gr, const ReduceArgs& a, uint32_t vec,
+                       cudaStream_t st) {
   HotGeom g;
   g.cols = t.dim < HOT_COLS ? t.dim : HOT_COLS;
   g.stride = (g.cols + 3u) & ~3u;
@@ -858,7 +890,7 @@ static void hot_launch(const TableDev& t, const OptimDev& op, const HyperDev& hy
     while (g.R < 64u && 2u * g.R * g.stride * 4u <= 32768u) g.R *= 2u;
     if (g.R * g.stride * 4u > 16384u) g.S = 6;  // 6 x 32 KB (the producers must not outnumber the slots)
   }
-  const size_t smem = (size_t)g.S * g.R * g.stride * 4u + (((size_t)t.dim + 3u) & ~(size_t)3u) * 4u;
+  const size_t smem = (size_t)g.S * g.R * g.stride * 4u;
   auto kern = k_reduce_hot<EPL, F16, SEND>;
   static size_t configured[64] = {0};  // per instantiation and device
   int dev = 0;
@@ -874,35 +906,51 @@ static void hot_launch(const TableDev& t, const OptimDev& op, const HyperDev& hy
   const uint32_t cap_blocks = cdiv(a.b.n, PB_WARM_MAX + 1);  // at most this many hot items exist
   uint32_t grid = 148u * per_sm;
   if (grid > cap_blocks) grid = cap_blocks ? cap_blocks : 1;
-  PB_LAUNCH_F(FAM_HOT, kern, grid, HOT_THREADS, smem, st, t, op, hy, sl, gr, a, g, g_hot_trace);
+  PB_LAUNCH_F(FAM_HOT, kern, grid, HOT_THREADS, smem, st, t, sl, gr, a, g, g_hot_trace);
+}
+
+// chain lanes own 2 columns (one or two chain warps) up to 128 columns, 4 above
+static bool hot_epl2(uint32_t dim) { return dim <= 128u && dim % 2u == 0; }
+
+uint32_t hot_stage_stride(uint32_t dim) { return (dim + 3u) & ~3u; }  // whole float4s for the chain lanes' stores
+
+void launch_reduce_hot(const TableDev& t, const SlotsDev& sl, const GradsDev& gr, bool f16, const ReduceArgs& a,
+                       cudaStream_t st, bool send) {
+  if (!a.b.n) return;
+  const uint32_t ev = f16 ? 8u : 4u;  // the producers' 16-byte loads need whole vectors and aligned rows
+  uint32_t hv = t.dim % ev == 0 ? 1u : 0u;
+  for (uint32_t s = 0; s < sl.n_slots && hv; ++s)
+    if (gr.ptr[s] && (reinterpret_cast<uintptr_t>(gr.ptr[s]) & 15u)) hv = 0;
+  if (getenv("PB_HOT_NO_VEC")) hv = 0;
+#define PB_H(E)                                                 \
+  if (send) {                                                   \
+    if (f16) hot_launch<E, true, true>(t, sl, gr, a, hv, st);   \
+    else hot_launch<E, false, true>(t, sl, gr, a, hv, st);      \
+  } else {                                                      \
+    if (f16) hot_launch<E, true, false>(t, sl, gr, a, hv, st);  \
+    else hot_launch<E, false, false>(t, sl, gr, a, hv, st);     \
+  }
+  if (hot_epl2(t.dim)) { PB_H(2) } else { PB_H(4) }
+#undef PB_H
+}
+
+void launch_step_hot(const TableDev& t, const OptimDev& op, const HyperDev& hy, const SlotsDev& sl, const GradsDev& gr,
+                     const ReduceArgs& a, cudaStream_t st) {
+  if (!a.b.n) return;
+  // a warp per item; blocks past the list's length (it lives on the device) return at once
+  uint32_t grid = cdiv(cdiv(a.b.n, PB_WARM_MAX + 1), 8u);
+  if (grid > 148u * 8u) grid = 148u * 8u;
+  if (hot_epl2(t.dim)) PB_LAUNCH(k_step_hot<2>, grid, 256, 0, st, t, op, hy, sl, gr, a);
+  else PB_LAUNCH(k_step_hot<4>, grid, 256, 0, st, t, op, hy, sl, gr, a);
 }
 
 void launch_reduce_items(const TableDev& t, const OptimDev& op, const HyperDev& hy, const SlotsDev& sl,
-                         const GradsDev& gr, bool f16, const ReduceArgs& a, cudaStream_t st, cudaStream_t st_hot,
-                         cudaStream_t st_warm, bool send) {
+                         const GradsDev& gr, bool f16, const ReduceArgs& a, cudaStream_t st, cudaStream_t st_warm,
+                         bool send) {
   if (!a.b.n) return;
   int vec, Gi;
   vec_group(t.dim, vec, Gi);
   uint32_t G = (uint32_t)Gi < 4u ? 4u : (uint32_t)Gi;
-  // hot items first in time when they have their own stream: they are the long poles
-  {
-    const uint32_t ev = f16 ? 8u : 4u;  // the producers' 16-byte loads need whole vectors and aligned rows
-    uint32_t hv = t.dim % ev == 0 ? 1u : 0u;
-    for (uint32_t s = 0; s < sl.n_slots && hv; ++s)
-      if (gr.ptr[s] && (reinterpret_cast<uintptr_t>(gr.ptr[s]) & 15u)) hv = 0;
-    if (getenv("PB_HOT_NO_VEC")) hv = 0;
-    // chain lanes own 2 columns (one or two chain warps) up to 128 columns, 4 above
-#define PB_H(E)                                                                 \
-  if (send) {                                                                   \
-    if (f16) hot_launch<E, true, true>(t, op, hy, sl, gr, a, hv, st_hot);       \
-    else hot_launch<E, false, true>(t, op, hy, sl, gr, a, hv, st_hot);          \
-  } else {                                                                      \
-    if (f16) hot_launch<E, true, false>(t, op, hy, sl, gr, a, hv, st_hot);      \
-    else hot_launch<E, false, false>(t, op, hy, sl, gr, a, hv, st_hot);         \
-  }
-    if (t.dim <= 128u && t.dim % 2u == 0) { PB_H(2) } else { PB_H(4) }
-#undef PB_H
-  }
   if (vec == 4) {
     if (f16) items_dispatch<4, true>(t, op, hy, sl, gr, a, G, st, st_warm, send);
     else items_dispatch<4, false>(t, op, hy, sl, gr, a, G, st, st_warm, send);

@@ -6,38 +6,61 @@ namespace pb {
 
 // ------------------------------------------------------------------------------------------------
 // A8 (NaN rule): a slot whose gradient holds any NaN is skipped whole (mod.rs:731-746).
-// grid.y = slot.  status[s] = tick when a NaN was seen (no reset needed between batches).
+// status[s] = tick when a NaN was seen (no reset needed between batches).
+//
+// A pure streaming read.  Each slot's gradient is cut into tiles of NAN_THREADS x NAN_LOADS 16-byte vectors; the grid
+// (a few blocks per SM) strides over the tiles of all slots, and a thread has the NAN_LOADS loads of its tile in flight
+// together.  The scan runs beside k_reduce_hot, one 256-thread block of <= 224 registers per SM, which leaves 8192
+// registers and no spare shared memory: __maxnreg__(32) keeps a scan block small enough to fit next to it.
+// A value is NaN iff its magnitude bits exceed those of inf, so one running unsigned max of the magnitudes (per 16-bit
+// half for f16: __vmaxu2) decides the whole tile.  Elements before the first 16-byte boundary of a slot and after the
+// last whole vector are checked one by one by the slot's first tile.
 // ------------------------------------------------------------------------------------------------
+constexpr uint32_t NAN_THREADS = 256;
+constexpr uint32_t NAN_LOADS = 4;  // 16-byte loads in flight per thread
+constexpr uint32_t NAN_TILE = NAN_THREADS * NAN_LOADS;  // vectors per tile
+
 template <bool F16>
-__global__ void __launch_bounds__(256) k_nan_scan(GradsDev gr, uint32_t elems_per_slot,
-                                                  const uint32_t* __restrict__ tick_ptr,
-                                                  uint32_t* __restrict__ nan_tick) {
-  uint32_t s = blockIdx.y;
-  const void* base = gr.ptr[s];
-  if (!base) return;
-  bool bad = false;
-  uint32_t stride = gridDim.x * blockDim.x;
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (F16) {
-    // 8 halves per 16 B load; every slot tensor is at least 16 B aligned (torch allocations are 512 B)
-    const uint4* p = reinterpret_cast<const uint4*>(base);
-    uint32_t nv = elems_per_slot / 8;
-    for (uint32_t j = i; j < nv; j += stride) {
-      uint4 v = p[j];
-      uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        uint32_t lo = w[k] & 0x7fffu, hi = (w[k] >> 16) & 0x7fffu;
-        bad |= (lo > 0x7c00u) | (hi > 0x7c00u);
+__global__ void __maxnreg__(32) k_nan_scan(GradsDev gr, uint32_t n_slots, uint32_t elems_per_slot, uint32_t tiles_per_slot,
+                                           const uint32_t* __restrict__ tick_ptr, uint32_t* __restrict__ nan_tick) {
+  constexpr uint32_t ES = F16 ? 2u : 4u, EV = 16u / ES;  // bytes per element, elements per vector
+  constexpr uint32_t MAG = F16 ? 0x7fff7fffu : 0x7fffffffu;
+  const uint32_t n_tiles = n_slots * tiles_per_slot;
+  for (uint32_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {  // (uniform over the block)
+    const uint32_t s = t / tiles_per_slot, tile = t - s * tiles_per_slot;
+    const unsigned char* base = reinterpret_cast<const unsigned char*>(gr.ptr[s]);
+    if (!base) continue;  // skipped slot: nothing to read
+    const uint32_t head = min(elems_per_slot, ((16u - (uint32_t)(reinterpret_cast<uintptr_t>(base) & 15u)) & 15u) / ES);
+    const uint32_t nv = (elems_per_slot - head) / EV;
+    const uint4* p = reinterpret_cast<const uint4*>(base + head * ES);
+    uint32_t m = 0;  // running max of the magnitudes
+    if (tile == 0) {  // the elements outside the whole vectors: [0, head) and [head + nv * EV, elems)
+      const uint32_t body_end = head + nv * EV;
+      for (uint32_t e = threadIdx.x; e < head + (elems_per_slot - body_end); e += NAN_THREADS) {
+        const uint32_t k = e < head ? e : body_end + (e - head);
+        const uint32_t x = F16 ? reinterpret_cast<const uint16_t*>(base)[k] : reinterpret_cast<const uint32_t*>(base)[k];
+        m = F16 ? __vmaxu2(m, x & 0x7fffu) : max(m, x & MAG);
       }
     }
-    const uint16_t* q = reinterpret_cast<const uint16_t*>(base);
-    for (uint32_t j = nv * 8 + i; j < elems_per_slot; j += stride) bad |= (q[j] & 0x7fffu) > 0x7c00u;
-  } else {
-    const float* p = reinterpret_cast<const float*>(base);
-    for (uint32_t j = i; j < elems_per_slot; j += stride) bad |= isnan(p[j]);
+    const uint32_t j0 = tile * NAN_TILE + threadIdx.x;
+    uint4 v[NAN_LOADS];
+#pragma unroll
+    for (uint32_t u = 0; u < NAN_LOADS; ++u) {
+      const uint32_t j = j0 + u * NAN_THREADS;
+      v[u] = j < nv ? p[j] : make_uint4(0u, 0u, 0u, 0u);
+    }
+#pragma unroll
+    for (uint32_t u = 0; u < NAN_LOADS; ++u) {
+      if (F16) {
+        m = __vmaxu2(m, __vmaxu2(__vmaxu2(v[u].x & MAG, v[u].y & MAG), __vmaxu2(v[u].z & MAG, v[u].w & MAG)));
+      } else {
+        m = max(m, max(max(v[u].x & MAG, v[u].y & MAG), max(v[u].z & MAG, v[u].w & MAG)));
+      }
+    }
+    const bool bad = F16 ? ((m & 0xffffu) > 0x7c00u || (m >> 16) > 0x7c00u)  // (h & 0x7fff) > 0x7c00: 0x7c00 is inf
+                         : m > 0x7f800000u;                                   // isnan
+    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) nan_tick[s] = *tick_ptr;
   }
-  if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) nan_tick[s] = *tick_ptr;
 }
 
 __global__ void k_slot_status(GradsDev gr, uint32_t n_slots, const uint32_t* __restrict__ tick_ptr,
@@ -96,12 +119,12 @@ __global__ void __launch_bounds__(256) k_update_direct(TableDev t, OptimDev op, 
 // ------------------------------------------------------------------------------------------------
 void launch_nan_scan(const GradsDev& gr, uint32_t n_slots, uint32_t elems_per_slot, bool f16, const uint32_t* tick,
                      uint32_t* nan_tick, int32_t* status, cudaStream_t st) {
-  uint32_t per = f16 ? elems_per_slot / 8 : elems_per_slot;
-  uint32_t gx = cdiv(per ? per : 1, 256 * 4);
-  if (gx > 148 * 4) gx = 148 * 4;
-  dim3 grid(gx, n_slots);
-  if (f16) PB_LAUNCH_F(FAM_NAN, k_nan_scan<true>, grid, 256, 0, st, gr, elems_per_slot, tick, nan_tick);
-  else PB_LAUNCH_F(FAM_NAN, k_nan_scan<false>, grid, 256, 0, st, gr, elems_per_slot, tick, nan_tick);
+  const uint32_t nv = elems_per_slot / (f16 ? 8u : 4u);
+  const uint32_t tiles_per_slot = nv ? cdiv(nv, NAN_TILE) : 1u;
+  uint32_t grid = n_slots * tiles_per_slot;
+  if (grid > 148u * 4u) grid = 148u * 4u;  // blocks stride over the tiles
+  if (f16) PB_LAUNCH_F(FAM_NAN, k_nan_scan<true>, grid, NAN_THREADS, 0, st, gr, n_slots, elems_per_slot, tiles_per_slot, tick, nan_tick);
+  else PB_LAUNCH_F(FAM_NAN, k_nan_scan<false>, grid, NAN_THREADS, 0, st, gr, n_slots, elems_per_slot, tiles_per_slot, tick, nan_tick);
   if (status) PB_LAUNCH(k_slot_status, 1, PB_MAX_SLOTS, 0, st, gr, n_slots, tick, nan_tick, status);
 }
 
